@@ -55,6 +55,9 @@ def parse():
     p.add_argument("--legs", default="all", help="secondary legs: all | none | comma list of amass,dual,ppo,tables")
     p.add_argument("--cpu-sample-envs", type=int, default=1024, help="envs of the in-line cpu_baseline sample (N=1 b200 arm)")
     p.add_argument("--no-cpu-baseline", action="store_true")
+    p.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to its caller (primary workload, "
+                   "rank 0) as DIR/<name>.npy, at most 64 MB (a seeded sample of envs above that): the same arguments give the same "
+                   "inputs, so two builds can be compared output for output")
     return p.parse_args()
 
 
@@ -539,6 +542,24 @@ def cpu_arm(envs, steps, warmup, procs=None):
     return envs * steps / dt, dt / steps * 1e3, procs
 
 
+DUMP_CAP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, outputs, n):
+    """outputs: per-env float32 arrays [n, ...] -> path/<name>.npy.  Above DUMP_CAP_BYTES in all, the same fixed, seeded sample of
+    env rows is written for every array, and its env ids as path/env_ids.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    row_bytes = sum(v.nbytes // n for v in outputs.values())
+    rows = min(n, (DUMP_CAP_BYTES - 4096 - 8 * n) // row_bytes)            # 4096: the .npy headers; 8 n: env_ids
+    if rows < n:
+        ids = np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+        outputs = {k: v[ids] for k, v in outputs.items()}
+        outputs["env_ids"] = ids.astype(np.float64)
+    for k, v in outputs.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 # ================================================================================================ main
 def main():
     args = parse()
@@ -604,10 +625,17 @@ def main():
         stats["resets"] += len(done)
         env.reset(done)
 
-    def step(i):
+    def step(i, snap=None):
         env.step(pool[i % len(pool)])                              # one graph replay
+        if snap is not None:                                       # --dump-outputs: the step's outputs before the reset rewrites them
+            for k, src in step_outputs().items():
+                snap[k].copy_(src)
         env.reset_done()                                           # reset(finished envs) from the device flags: mask + one graph replay
         # (step + reset captured as ONE graph measured 1.4 % slower than the two replays, profiles/r2z_notes.md: not kept)
+
+    def step_outputs():
+        return {"obs": env.obs_buf, "rew": env.rew_buf, "reset": env.reset_buf, "terminate": env.extras["terminate"],
+                "sub_rewards": env.extras["sub_rewards"]}
     for i in range(4):
         step_ids(i)
     env.enable_cuda_graph(count_nodes=True)
@@ -629,13 +657,22 @@ def main():
     prof = os.environ.get("B200_BENCH_PROFILE") == "1"      # tools/federer_launches.sh: ncu --profile-from-start off sees the timed loop only
     if prof:
         torch.cuda.cudart().cudaProfilerStart()
-    step_ms = timed_steps(step, K, flush, sampler)
+    dump = args.dump_outputs and rank == 0
+    snap = {k: torch.empty_like(v) for k, v in step_outputs().items()} if dump else None
+    timed_step = (lambda i: step(i, snap if i == K - 1 else None)) if dump else step
+    step_ms = timed_steps(timed_step, K, flush, sampler)
     barrier()
     if prof:
         torch.cuda.cudart().cudaProfilerStop()
     wall = time.perf_counter() - t_wall
     clocks = sampler.stop()
     total_ms = sum(step_ms)
+    # what the caller of the timed path receives from its last step: the step's outputs (taken before reset_done clears the flags of
+    # the finished envs) and the observation after the reset, the one the policy sees next
+    outputs = None
+    if dump:
+        snap["obs_after_reset"] = env.obs_buf
+        outputs = {k: v.detach().float().cpu().numpy() for k, v in snap.items()}
     # the physics launch alone (dominant kernel): the SAME rollout continued for 10 steps with the step run eagerly (an event pair
     # inside b200env_step cannot live in a graph), L2 flushed before every step as in the timed loop
     g_saved, env._graph = env._graph, None
@@ -810,6 +847,8 @@ def main():
                                              "logic + fp32 policy MLP + float64 articulated step with ball); `--impl reference` runs all envs"}
         except Exception as ex:
             out["cpu_baseline"] = {"value": None, "unit": "env-steps/s", "cores": None, "kind": "port", "sample": "failed: " + repr(ex)[:200]}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs, N)
     emit(out)
     if world > 1:
         dist.destroy_process_group()

@@ -65,23 +65,17 @@ def test_no_gpu_means_loud_failure():
 
 
 def test_shim_quaternion_helpers_match_poselib_conventions():
-    """the only foreign arithmetic of the oracle (isaacgym.torch_utils) is cross-checked against the
-    reference's own poselib definitions when the reference tree is present, else against closed forms"""
+    """the only foreign arithmetic of the oracle (isaacgym.torch_utils) is cross-checked against the reference's own poselib
+    definitions (their outputs on seeded inputs, tests/golden/poselib_quat.npz) and against closed forms"""
     import sys
     sys.path.insert(0, os.path.join(ROOT, "vid2player3d_b200", "shim"))
     from isaacgym import torch_utils as IG
-    g = torch.Generator().manual_seed(0)
-    a = torch.nn.functional.normalize(torch.randn(64, 4, generator=g), dim=-1)
-    b = torch.nn.functional.normalize(torch.randn(64, 4, generator=g), dim=-1)
-    v = torch.randn(64, 3, generator=g)
-    if os.path.isdir("/root/reference/poselib"):
-        sys.path.insert(0, "/root/reference/poselib")
-        from poselib.core import rotation3d as P
-        assert torch.allclose(IG.quat_mul(a, b), P.quat_mul(a, b), atol=1e-6)
-        assert torch.allclose(IG.quat_conjugate(a), P.quat_conjugate(a))
-        ang = torch.rand(64, generator=g) * 6 - 3
-        assert torch.allclose(IG.quat_from_angle_axis(ang, v), P.quat_from_angle_axis(ang, v), atol=1e-6)
-        assert torch.allclose(IG.quat_rotate(a, v), P.quat_rotate(a, v), atol=1e-5)
+    P = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(ROOT, "tests", "golden", "poselib_quat.npz")).items()}
+    a, b, v, ang = P["a"], P["b"], P["v"], P["ang"]
+    assert torch.allclose(IG.quat_mul(a, b), P["quat_mul"], atol=1e-6)
+    assert torch.allclose(IG.quat_conjugate(a), P["quat_conjugate"])
+    assert torch.allclose(IG.quat_from_angle_axis(ang, v), P["quat_from_angle_axis"], atol=1e-6)
+    assert torch.allclose(IG.quat_rotate(a, v), P["quat_rotate"], atol=1e-5)
     # closed forms
     ident = torch.tensor([[0.0, 0, 0, 1]]).repeat(64, 1)
     assert torch.allclose(IG.quat_mul(a, IG.quat_conjugate(a)), ident, atol=1e-6)
@@ -161,9 +155,7 @@ def test_left_handed_asset_in_canonical_order():
 
 
 def test_model_compiler_reproduces_committed_blob():
-    ref = "/root/reference/embodied_pose/data/assets/mjcf/smpl_mesh_humanoid_amass_v1.xml"
-    if not os.path.exists(ref):
-        pytest.skip("reference assets not present on this box")
+    ref = os.path.join(ROOT, "tests", "golden", "amass_asset", "mjcf", "smpl_mesh_humanoid_amass_v1.xml")   # the reference's asset
     from vid2player3d_b200 import model_compiler
     a = model_compiler.compile_mjcf(ref)
     b = model_compiler.load_compiled("smpl_mesh_humanoid_amass_v1")
@@ -226,25 +218,51 @@ def test_vec_task_and_parse_task_surface():
         pt(A, {"env": {}}, {}, None)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/embodied_pose"), reason="reference checkout not present (GPU box)")
 def test_reference_config_module_runs_on_the_shim():
-    """Level B of the boundary (SURVEY.md 8b): the reference's own utils/config.py (get_args / load_cfg / parse_sim_params)
-    imports and runs UNCHANGED against vid2player3d_b200/shim/isaacgym, in a subprocess so sys.modules stays clean."""
+    """Level B of the boundary (SURVEY.md 8b): what the reference's own utils/config.py (get_args / load_cfg / parse_sim_params,
+    amass_im at 64 envs) hands vid2player3d_b200/shim/isaacgym.  Its inputs to the shim - the custom parameters and command line
+    of `gymutil.parse_arguments`, the yaml sim section of `gymutil.parse_sim_config` - and the SimParams fields it ended with were
+    recorded from one run of it (tests/golden/make_golden_host.py -> tests/golden/ref_callers.json).  Replayed here in a subprocess
+    (sys.modules / sys.argv stay clean): the parsed arguments follow the command line and the parameters' defaults, the Isaac Gym
+    defaults the module reads next are set, the sim section lands in SimParams, and every SimParams field the module assigns exists
+    on the shim's classes.  The module itself is not part of this repository and is not run."""
     code = r'''
-import sys
-sys.path.insert(0, "%s/vid2player3d_b200/shim"); sys.path.insert(0, "/root/reference/embodied_pose")
-sys.argv = ["run.py", "--cfg", "amass_im", "--headless", "--num_envs", "64"]
-from isaacgym import gymapi
-from utils.config import get_args, load_cfg, parse_sim_params
-import os; os.chdir("/root/reference")
-args = get_args()
-cfg, cfg_train = load_cfg(args)
-sp = parse_sim_params(args, cfg, cfg_train)
-assert abs(sp.dt - 1.0 / 60.0) < 1e-9 and sp.substeps == cfg["sim"]["substeps"] == 2, (sp.dt, sp.substeps)
-assert sp.physx.num_position_iterations == 4 and sp.physx.contact_offset == 0.02, (sp.physx.num_position_iterations,)
-assert cfg["env"]["numEnvs"] == 64 and cfg["name"] == "HumanoidSMPLIM"
-print("OK", args.task, sp.up_axis == gymapi.UP_AXIS_Z)
-''' % ROOT
+import json, sys
+sys.path.insert(0, "%s/vid2player3d_b200/shim")
+from isaacgym import gymapi, gymutil
+rec = json.load(open("%s/tests/golden/ref_callers.json"))["config"]
+pa = rec["parse_arguments"]
+types = {"str": str, "int": int, "float": float}
+params = [{k: (types[v] if k == "type" else v) for k, v in p.items()} for p in pa["custom_parameters"]]
+argv = pa["argv"]
+sys.argv = ["run.py"] + argv
+args = vars(gymutil.parse_arguments(custom_parameters=params, **pa["kwargs"]))
+for p in params:
+    dest, flag = p["name"][2:], p.get("action") == "store_true"
+    if p["name"] in argv:
+        want = True if flag else p["type"](argv[argv.index(p["name"]) + 1])
+    else:
+        want = p.get("default", False if flag else None)
+    assert args[dest] == want, (dest, args[dest], want)
+assert args["num_envs"] == 64 and args["headless"] is True and args["cfg"] == "amass_im"
+# Isaac Gym's parse_arguments defaults without --sim_device / --pipeline / --flex, read by get_args and parse_sim_params
+assert (args["sim_device_type"], args["compute_device_id"], args["use_gpu_pipeline"], args["use_gpu"]) == ("cuda", 0, True, True)
+assert args["physics_engine"] == gymapi.SIM_PHYSX and args["slices"] == args["subscenes"] == 0 and args["num_threads"] == 0
+sim_cfg = rec["parse_sim_config"]["sim_cfg"]
+sp = gymapi.SimParams()
+gymutil.parse_sim_config(sim_cfg, sp)
+for k, v in sim_cfg.items():
+    if k in ("physx", "flex"):
+        for kk, vv in v.items():
+            assert getattr(getattr(sp, k), kk) == vv, (k, kk)
+    else:
+        assert getattr(sp, k) == v, k
+want = rec["sim_params"]
+fresh = gymapi.SimParams()
+assert set(want) - {"physx", "flex"} <= set(vars(fresh)), set(want) - set(vars(fresh))
+assert set(want["physx"]) <= set(vars(fresh.physx)) and set(want["flex"]) <= set(vars(fresh.flex))
+print("OK")
+''' % (ROOT, ROOT)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0 and "OK" in r.stdout, r.stdout[-2000:] + r.stderr[-3000:]
 
@@ -353,24 +371,28 @@ def test_motion_lib_formats_directory_and_merge(tmp_path):
         ML.FlatMotionLib.load_any(str(empty))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/embodied_pose"), reason="reference checkout not present (GPU box)")
-def test_from_reference_motion_lib_pickle(tmp_path):
+def test_from_reference_motion_lib_pickle():
     """a reference `torch.save(motion_lib)` pickle (what every reference yaml's motion_file names) loads through
-    FlatMotionLib.load_any / from_reference; run in a subprocess with the reference importable, like the reference's own torch.load"""
+    FlatMotionLib.load_any / from_reference.  The pickle (tests/golden/ref_motion_lib.pth) was written by the reference's
+    MotionLib from the synthetic library rebuilt below (tests/golden/make_golden_host.py); it is loaded in a subprocess with a
+    stand-in for the reference's `utils.motion_lib.MotionLib` class (unpickling restores the instance attributes only)."""
     code = r'''
-import os, sys
-sys.path.insert(0, os.path.join(%(root)r, "tests", "golden")); sys.path.insert(0, %(root)r)
+import os, sys, types
+sys.path.insert(0, %(root)r)
 import numpy as np, torch
-import make_golden as G                     # builds a reference MotionLib object from a synthetic flat library
+from vid2player3d_b200 import model_compiler, motion_lib
 from vid2player3d_b200.motion_lib import FlatMotionLib
-model, flat, key = G.small_lib()
-ml = G.make_ref_motion_lib(flat, key, model["dof_body_ids"])
-path = os.path.join(%(tmp)r, "lib.pth")
-torch.save(ml, path)
-back = FlatMotionLib.load_any(path)
+sys.modules["utils"] = types.ModuleType("utils")
+sys.modules["utils.motion_lib"] = ml_mod = types.ModuleType("utils.motion_lib")
+ml_mod.MotionLib = type("MotionLib", (), {})
+model = model_compiler.load_compiled("smpl_mesh_humanoid_amass_v1")
+flat = motion_lib.synthetic(model, num_motions=3, num_frames=12, seed=11, sigma=0.08, ragged=True)
+flat.min_verts_h = np.linspace(-0.02, 0.03, 3).astype(np.float32)
+flat.motion_bodies = np.random.default_rng(5).normal(size=(3, 11)).astype(np.float32)
+back = FlatMotionLib.load_any(os.path.join(%(root)r, "tests", "golden", "ref_motion_lib.pth"))
 for k in FlatMotionLib.FIELDS:
     assert np.array_equal(np.asarray(getattr(back, k)), np.asarray(getattr(flat, k))), k
 print("ok")
-''' % {"root": ROOT, "tmp": str(tmp_path)}
+''' % {"root": ROOT}
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0 and r.stdout.strip().endswith("ok"), r.stdout[-1500:] + r.stderr[-2500:]
